@@ -2,6 +2,7 @@
 """Benchmark of the DM-NeRF render hot path (BASELINE.json metric: rays/sec, 64 coarse + 128 fine samples).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--scaling weak|strong]
+                    [--dump-outputs DIR]
 
 One "step" = one full 640x480 synthetic frame (307 200 rays) per GPU through the complete pipeline
 (coarse net -> composite -> importance sampling -> fine net -> composite, object head included), i.e.
@@ -24,6 +25,10 @@ on every rank; `value` = frame rays / max-over-ranks time, `allgather` = that co
 
 --impl reference times that same CPU path alone (the reference is pure Python/torch and cannot travel to the GPU
 box; the oracle is its bit-for-bit restatement, see oracle/dmnerf_oracle.py).
+
+--dump-outputs DIR writes the per-ray maps the last timed step returned (rgb_fine, depth_fine, acc_fine, ins_fine) as
+DIR/<name>.npy in float32, so that two builds run with the same arguments (same seeded weights and rays) can be compared
+map by map.  Above 60 MiB in all, every map keeps the same seeded sample of rays.
 """
 import argparse
 import json
@@ -58,6 +63,7 @@ def parse():
     ap.add_argument("--cpu-procs", type=int, default=0,
                     help="cpu_baseline: also run this many concurrent CPU workers (whole-box figure); 0 = cores // 16")
     ap.add_argument("--cpu-worker", type=int, default=0, help=argparse.SUPPRESS)    # internal: one whole-box worker, N threads
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's per-ray maps as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -266,6 +272,27 @@ class ClockSampler:
                 "reasons": reasons}
 
 
+# --------------------------------------------------------------------------------------------- outputs
+DUMP_BYTES = 60 << 20          # keeps a dump below 64 MB with room for the .npy headers
+
+
+def dump_outputs(out, n_rays, ins_num, path):
+    """Write one step's result as path/<map>.npy (float32).  `out` is render_rays' dict of per-ray maps, or on N > 1 ranks
+    the all-gathered [N, rays, 5 + ins_num] image slab, whose first `n_rays` rows are unpacked into the same maps.  When the
+    maps exceed DUMP_BYTES they all keep the same rays: a sorted sample drawn from a fixed seed."""
+    from dmnerf_b200.parallel import unpack_image
+    if torch.is_tensor(out):
+        out = unpack_image(out.reshape(-1, out.shape[-1])[:n_rays], ins_num)
+    maps = {k: v.float().contiguous().cpu().numpy() for k, v in out.items()}
+    total = sum(a.nbytes for a in maps.values())
+    if total > DUMP_BYTES:
+        keep = np.random.Generator(np.random.PCG64(0)).choice(n_rays, DUMP_BYTES * n_rays // total, replace=False)
+        maps = {k: a[np.sort(keep)] for k, a in maps.items()}
+    os.makedirs(path, exist_ok=True)
+    for k, a in maps.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 # --------------------------------------------------------------------------------------------- our arm
 def run_ours(args):
     import ctypes as C
@@ -351,7 +378,10 @@ def run_ours(args):
         for s in range(args.steps):
             flush.fill_(s & 0xFF)
             evs[s][0].record()
-            step_device()
+            if s + 1 < args.steps:
+                step_device()
+            else:
+                last = step_device()             # only the last step's result is kept, for --dump-outputs
             evs[s][1].record()
             ms = (C.c_float * 6)()
             _lib.check(lib.dmnerf_profile_read(ctx.handle, ms, 6), "profile_read")
@@ -367,6 +397,9 @@ def run_ours(args):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         dev_ms = float(t.item())
         gather_ms = sum(a.elapsed_time(b) for a, b in gather_ev) if gather_ev else 0.0
+        if args.dump_outputs and rank == 0:
+            dump_outputs(last, n_rays * (1 if strong else world), ins_num, args.dump_outputs)
+        del last
 
         # ---- end to end through the C ABI with HOST buffers (pinned), H2D + D2H inside the timed region
         h = {k: torch.empty(shape, dtype=torch.float32).pin_memory() for k, shape in

@@ -91,21 +91,55 @@ def test_dropin_networks_package_exposes_reference_names():
     assert r.returncode == 0 and "ok" in r.stdout, r.stderr
 
 
-def test_dropin_rebinds_native_functions_inside_the_reference_modules():
+# A stand-in for a DM-NeRF checkout's networks/ package: the module and function names the drop-in resolves, each function
+# returning the callees it finds through its own module globals, and the same cross-module import lines as the original
+# (manipulator and tester import from networks.helpers / networks.evaluator / networks.render).
+STAND_IN_NETWORKS = {
+    "helpers.py": """
+def get_rays_k(H, W, K, c2w): return "stand-in"
+def get_select_full(*args): return get_rays_k
+def get_select_crop(*args): return get_rays_k
+def z_val_sample(*args): return "stand-in"
+def sample_pdf(*args): return "stand-in"
+def get_rays(*args): return get_rays_k, sample_pdf
+""",
+    "evaluator.py": """
+def hungarian(*args): return "stand-in"
+def ins_criterion(*args): return hungarian
+def to8b(x): return x
+def calculate_ap(*args): return "stand-in"
+def ins_eval(*args): return hungarian
+""",
+    "manipulator.py": """
+from networks.evaluator import to8b, ins_eval
+from networks.helpers import get_rays_k, sample_pdf
+def exchanger(*args): return "stand-in"
+def manipulator_render(*args): return "stand-in"
+def manipulator_nerf(*args): return "stand-in"
+def manipulator(*args): return manipulator_nerf, manipulator_render, exchanger
+def manipulator_eval(*args): return manipulator, exchanger, get_rays_k, sample_pdf
+def manipulator_demo(*args): return manipulator, exchanger, get_rays_k, sample_pdf
+""",
+    "tester.py": """
+from networks.render import dm_nerf
+from networks.evaluator import to8b, ins_eval
+from networks.helpers import get_rays_k, z_val_sample
+def render_test(*args): return dm_nerf, get_rays_k, z_val_sample
+""",
+}
+
+
+def test_dropin_rebinds_native_functions_inside_the_reference_modules(tmp_path):
     """The reference drivers (manipulator_eval / manipulator_demo, get_select_*; train_*.py through networks.evaluator)
     resolve their callees through their OWN module globals: the drop-in must rebind the native functions there, not only
-    re-export them (build container only: needs the reference checkout)."""
-    ref = "/root/reference"
-    if not os.path.isdir(os.path.join(ref, "networks")):
-        pytest.skip("reference checkout not present")
-    env = dict(os.environ, DMNERF_REFERENCE_ROOT=ref,
-               PYTHONPATH=os.pathsep.join([os.path.join(ROOT, "dm-nerf_b200", "dropin"), ROOT, ref]))
+    re-export them.  DMNERF_REFERENCE_ROOT points at a stand-in checkout with the reference's module layout."""
+    ref = tmp_path / "reference"
+    (ref / "networks").mkdir(parents=True)
+    for name, src in STAND_IN_NETWORKS.items():
+        (ref / "networks" / name).write_text(src)
+    env = dict(os.environ, DMNERF_REFERENCE_ROOT=str(ref),
+               PYTHONPATH=os.pathsep.join([os.path.join(ROOT, "dm-nerf_b200", "dropin"), ROOT]))
     code = r"""
-import sys, types
-for name in ("lpips", "cv2", "imageio", "skimage", "skimage.metrics", "h5py", "configargparse", "matplotlib", "matplotlib.pyplot", "open3d", "trimesh"):
-    m = types.ModuleType(name); sys.modules[name] = m
-sys.modules["skimage"].metrics = sys.modules["skimage.metrics"]
-sys.modules["matplotlib"].pyplot = sys.modules["matplotlib.pyplot"]
 import dmnerf_b200.manipulator as nm, dmnerf_b200.helpers as nh, dmnerf_b200.evaluator as ne, dmnerf_b200.render as nr
 import networks.manipulator as M, networks.helpers as H, networks.evaluator as E
 assert M.manipulator is nm.manipulator and M.exchanger is nm.exchanger
@@ -113,14 +147,16 @@ for fn in (M.manipulator_eval, M.manipulator_demo):
     g = fn.__globals__
     assert g["manipulator"] is nm.manipulator and g["exchanger"] is nm.exchanger, fn
     assert g["get_rays_k"] is nh.get_rays_k and g["sample_pdf"] is nh.sample_pdf, fn
+    assert fn() == (nm.manipulator, nm.exchanger, nh.get_rays_k, nh.sample_pdf), fn
 assert H.get_select_full is nh.get_select_full and H.get_select_crop is nh.get_select_crop and H.get_rays_k is nh.get_rays_k
-assert H.rotation_x.__globals__["get_rays_k"] is nh.get_rays_k if hasattr(H, "rotation_x") else True
+assert H.get_rays() == (nh.get_rays_k, nh.sample_pdf)      # a reference helper the drop-in keeps calls the native callees
 assert E.ins_criterion is ne.ins_criterion and callable(E.ins_eval) and callable(E.calculate_ap)
 import networks.tester as T                       # the reference's test loop, resolved through the package __path__
 assert T.dm_nerf is nr.dm_nerf and T.get_rays_k is nh.get_rays_k and T.z_val_sample is nh.z_val_sample
+assert T.render_test() == (nr.dm_nerf, nh.get_rays_k, nh.z_val_sample)
 print("ok")
 """
-    r = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, cwd="/tmp")
+    r = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, cwd=str(tmp_path))
     assert r.returncode == 0 and "ok" in r.stdout, r.stderr[-3000:]
 
 
